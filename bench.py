@@ -56,7 +56,14 @@ def parse():
     ap.add_argument("--scaling", default="strong", choices=["strong", "weak"],
                     help="N>1: strong = the named config sharded over N GPUs (BASELINE config #4); weak = the world, the entities and "
                          "the subscribers grow N-fold in X (per-GPU work fixed)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (the results a caller of the tick receives) as DIR/<name>.npy, "
+                         "float64, at most 60 MB in all: lists the library returns as sets in sorted row order, larger arrays as a fixed, seeded "
+                         "sample of rows.  N>1: one set of files per rank (rank<r>_<name>.npy)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm only counts queries, it keeps no results")
+    return args
 
 
 def world_config(args):
@@ -222,6 +229,89 @@ def pinned(shape, dtype):
 
     t = torch.empty(shape, dtype=dtype, pin_memory=True)
     return t, t.numpy()
+
+
+DUMP_BYTES = 60_000_000  # --dump-outputs, all files of all ranks (under 64 MB with room to spare)
+
+
+def _fair_caps(sizes, budget):
+    """Per-array value caps within `budget`: equal shares, and what a smaller array leaves of its share goes to the larger ones."""
+    caps, left = {}, budget
+    for i, (k, n) in enumerate(sorted(sizes.items(), key=lambda kv: kv[1])):
+        caps[k] = min(n, left // (len(sizes) - i))
+        left -= caps[k]
+    return caps
+
+
+def _sample_rows(n, k):
+    """The fixed, seeded sample of k of n rows, in row order: the same rows in every run with the same n."""
+    return np.arange(n) if k >= n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+
+
+def _sorted_rows(a):
+    return a[np.lexsort(a.T[::-1])]
+
+
+class _DeviceArray:
+    """A device array of the library, for torch.as_tensor."""
+
+    def __init__(self, address, n, typestr):
+        self.__cuda_array_interface__ = {"shape": (n,), "typestr": typestr, "data": (address, False), "version": 2}
+
+
+def dump_outputs(e, dirname, S, sm, dev, prefix, budget_bytes):
+    """--dump-outputs: the results of the engine's last tick as float64 .npy files, for comparing two builds output for output.
+    Everything chd_fetch_results returns, plus the expanded visible list (vis_entity) that stays in HBM.  All values are integers
+    below 2^53, so float64 holds them exactly; a due record is its twelve 32-bit words (64-bit fields as low, high).  The interest
+    diff, the due list and the handover list are sets (include/chd_gpu.h) and are written in sorted row order.  An array larger
+    than its share of the budget is a fixed, seeded sample of its rows (_sample_rows)."""
+    import torch
+
+    from channeld_b200 import capi
+
+    def u32(n):
+        return np.zeros(int(n), np.uint32)
+
+    P, D, H = int(sm.n_pairs), max(int(sm.n_sub_new), int(sm.n_unsub)), int(sm.n_handover)
+    b = dict(pair_off=u32(S + 1), pair_channel=u32(P), pair_dist=u32(P), pair_interval_ms=u32(P), new_sub=u32(D), new_channel=u32(D),
+             unsub_sub=u32(D), unsub_channel=u32(D), due=np.zeros(int(sm.n_due), capi.DUE_DTYPE), handover_entity=u32(H),
+             handover_src=u32(H), handover_dst=u32(H), query_status=u32(S), vis_off=np.zeros(S + 1, np.uint64),
+             cell_start=u32(e.n_cells + 1), sorted_entity=u32(sm.n_entities_in_world))
+    rb = capi.ResultBuffers()
+    for k, a in b.items():
+        setattr(rb, k, capi.ptr(a))
+    rb.pair_cap, rb.diff_cap, rb.due_cap, rb.handover_cap, rb.status_cap, rb.entity_cap = P, D, int(sm.n_due), H, S, int(sm.n_entities_in_world)
+    got = capi.TickSummary()
+    e._ck(e.L.chd_fetch_results(e.h, C.byref(rb), C.byref(got)))
+    nn, nu = int(got.n_sub_new), int(got.n_unsub)
+    out = {
+        "summary": np.array(list(got.as_dict().values()), np.uint64),  # chd_tick_summary, in field order
+        "query_status": b["query_status"],
+        "pair_off": b["pair_off"],
+        "pairs": np.stack([b["pair_channel"], b["pair_dist"], b["pair_interval_ms"]], 1),
+        "sub_new": _sorted_rows(np.stack([b["new_sub"][:nn], b["new_channel"][:nn]], 1)),
+        "unsub": _sorted_rows(np.stack([b["unsub_sub"][:nu], b["unsub_channel"][:nu]], 1)),
+        "due": _sorted_rows(b["due"].view(np.uint32).reshape(-1, 12)),
+        "handover": _sorted_rows(np.stack([b["handover_entity"], b["handover_src"], b["handover_dst"]], 1)),
+        "vis_off": b["vis_off"],
+        "cell_start": b["cell_start"],
+        "sorted_entity": b["sorted_entity"],
+    }
+    V = int(got.n_visible)
+    sizes = dict({k: a.size for k, a in out.items()}, vis_entity=V)
+    caps = _fair_caps(sizes, budget_bytes // 8 - 16 * len(sizes))  # 128 bytes of .npy header per file
+    out["vis_entity"] = u32(0)
+    if V:
+        vis = torch.as_tensor(_DeviceArray(e.device_view(capi.VIEW_VIS_ENTITY)[0], V, "<i4"), device=dev)
+        rows = torch.from_numpy(_sample_rows(V, caps["vis_entity"])).to(dev)
+        out["vis_entity"] = vis[rows].cpu().numpy().view(np.uint32)
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in out.items():
+        if a.size > caps[k]:
+            a = a[_sample_rows(len(a), caps[k] // (a.size // len(a)))]
+        np.save(os.path.join(dirname, prefix + k + ".npy"), a.astype(np.float64))
+    sampled = ["%s %d of %d" % (k, caps[k], n) for k, n in sizes.items() if n > caps[k]]
+    print("[bench] outputs of the last timed step in %s (sampled values: %s)" % (dirname, ", ".join(sampled) or "none"), file=sys.stderr)
 
 
 def run_ours(args):
@@ -450,6 +540,8 @@ def run_ours(args):
         sm = e.summary()  # raises on any capacity overflow during the timed steps
         ek_tot, ek_n = e.profile_get(capi.STAGE_EMIT_KERNEL)
         emit_kernel_ms_timed = ek_tot / max(ek_n, 1)
+        if args.dump_outputs:  # before the passes below overwrite the last timed step's results
+            dump_outputs(e, args.dump_outputs, S, sm, dev, "rank%d_" % rank if world > 1 else "", DUMP_BYTES // world)
         e.profile_enable(True)  # instrumented pass (not timed): every stage, same inputs
         for i in range(n_prof):
             step(args.warmup + 1 + args.steps + i, dev_in, batches_dev, rings_dev)

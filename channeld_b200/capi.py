@@ -121,6 +121,8 @@ SYMBOLS = [
     "chd_add_subscribers", "chd_remove_subscribers", "chd_fetch_results_async", "chd_fetch_wait", "chd_rings_init", "chd_rings_append", "chd_get_rings", "chd_set_channel_start_times", "chd_set_payload_bytes", "chd_assemble_payloads", "chd_frame_packets", "chd_comm_unique_id", "chd_comm_init", "chd_comm_info", "chd_comm_destroy", "chd_tick_sharded", "chd_collective_count", "chd_comm_exchange_mode", "chd_comm_use_collective", "chd_migrate_out", "chd_migrate_in", "chd_get_rehome",
 ]
 STAGE_BUILD, STAGE_INTEREST, STAGE_EMIT, STAGE_EMIT_KERNEL, STAGE_FANOUT, STAGE_TICK, STAGE_EXPORT, STAGE_EXCHANGE, STAGE_IMPORT, STAGE_READBACK = range(10)
+(VIEW_CELL_START, VIEW_SORTED_ENTITY, VIEW_ENT_CELL, VIEW_PAIR_OFF, VIEW_PAIR_CHANNEL, VIEW_PAIR_DIST, VIEW_VIS_OFF, VIEW_VIS_ENTITY,
+ VIEW_DUE) = range(9)  # chd_device_view
 
 _lib = None
 
