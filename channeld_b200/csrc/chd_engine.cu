@@ -5,7 +5,7 @@ static thread_local std::string g_create_error;
 
 // epochs start at 1 so that the zero-initialised descriptors (epoch 0) read as stale on first use
 bool chd_init_epochs(chd_engine* e) {
-    const unsigned long long ones[8] = {1, 1, 1, 1, 1, 1, 1, 1};
+    const unsigned long long ones[EP_COUNT] = {1, 1, 1, 1, 1, 1, 1, 1, 1};
     return cudaMemcpy(e->d_epoch, ones, sizeof ones, cudaMemcpyHostToDevice) == cudaSuccess;
 }
 
@@ -302,7 +302,7 @@ chd_status chd_create(const chd_grid_cfg* cfg, const chd_limits* lim_in, int dev
          dalloc(e, &e->d_prev_key, N) && dalloc(e, &e->d_tmp_key, N) && dalloc(e, &e->d_tmp_val, N) &&
          dalloc(e, &e->d_sorted_key, N) && dalloc(e, &e->d_sorted4, 4 * (((N + 3) / 4) * 4 + 8)) && dalloc(e, &e->d_cell_start, C + 2) &&
          dalloc(e, &e->d_hist, (uint64_t)BUILD_MAX_BINS * e->build_blocks + 2) &&
-         dalloc(e, &e->d_epoch, 8) && chd_init_epochs(e) &&
+         dalloc(e, &e->d_epoch, EP_COUNT) && chd_init_epochs(e) &&
          chd_make_site(e, e->site_hist, (uint64_t)BUILD_MAX_BINS * e->build_blocks + 1, EP_BUILD) &&
          chd_make_site(e, e->site_hist_b, (uint64_t)BUILD_MAX_BINS * e->build_blocks + 1, EP_BUILD) &&
          chd_make_site(e, e->site_qoff, Q + 1, EP_QUERY) && chd_make_site(e, e->site_slot, S + 1, EP_QUERY) &&

@@ -93,7 +93,7 @@ struct chd_engine {
     // one look-back scan site per call site: stages run concurrently on two streams and must not share scan state
     unsigned long long* d_epoch = nullptr;  // [EP_COUNT] stage epochs for the look-back scans
     ScanSite site_hist_b{}, site_pchist_b{}, site_hist{}, site_qoff{}, site_slot{}, site_pchist{}, site_voff{}, site_border{};
-    uint64_t stage_execs[8] = {};
+    uint64_t stage_execs[9] = {};  // [EP_COUNT]
     std::vector<ScanSite*> sites;  // every scan site (chd_make_site registers them)
     uint32_t build_blocks = 0;
     bool assigned = false, built = false, have_prev_key = false, entities_dirty = false;
@@ -263,6 +263,26 @@ struct chd_engine {
     // scratch of the tick driver's getters (chd_get_visible*, export counts): separate from h_u32, which the stateless entry
     // points use under the engine mutex from other threads
     uint32_t* h_get = nullptr;
+    // ---- per-subscriber visibility deltas (chd_visdelta.cu): allocated by chd_visible_delta_enable
+    bool slab_set = false;              // chd_set_slab was called: entity indices are not stable across ticks
+    bool assigned_since_build = false;  // d_key no longer holds the cell keys of the last build
+    struct VisDelta {
+        bool on = false, called = false;
+        uint64_t cap = 0;                  // entries of each output list
+        uint32_t S_out = 0, S_call = 0;    // slots in the output CSR / current slot count of the last call
+        uint32_t S_bound = 0, n_bound = 0; // host upper bounds of the baseline's slot and entity counts
+        uint32_t nb = 1, per_block = 0;    // mover sort geometry
+        VdState* d_state = nullptr;
+        uint32_t *d_base_key = nullptr, *d_base_cs = nullptr, *d_base_sorted = nullptr, *d_base_off = nullptr, *d_base_cell = nullptr,
+                 *d_base_sub = nullptr;
+        uint32_t *d_mv_ent = nullptr, *d_mv_dkey = nullptr, *d_mv_skey = nullptr, *d_tmp_key = nullptr, *d_tmp_val = nullptr,
+                 *d_dst_key = nullptr, *d_dst_ent = nullptr, *d_src_key = nullptr, *d_src_ent = nullptr, *d_dst_start = nullptr,
+                 *d_src_start = nullptr, *d_hist = nullptr;
+        uint32_t *d_ecnt = nullptr, *d_lcnt = nullptr;
+        uint64_t *d_epoff = nullptr, *d_lpoff = nullptr, *d_enter_off = nullptr, *d_leave_off = nullptr;
+        uint32_t *d_enter = nullptr, *d_leave = nullptr;
+        ScanSite site_mv{}, site_h[4]{}, site_e{}, site_l{};
+    } vd;
 
     bool fail(const char* fmt, ...) const {
         char buf[512];
@@ -325,7 +345,8 @@ static bool dalloc(chd_engine* e, T** p, uint64_t count) {
     return true;
 }
 
-enum { EP_BUILD = 0, EP_QUERY, EP_EMIT, EP_FANOUT, EP_BORDER, EP_BCAST, EP_CLASS, EP_PAYLOAD, EP_COUNT };  // d_epoch has 8 slots
+enum { EP_BUILD = 0, EP_QUERY, EP_EMIT, EP_FANOUT, EP_BORDER, EP_BCAST, EP_CLASS, EP_PAYLOAD, EP_DELTA, EP_COUNT };  // d_epoch has EP_COUNT slots
+static_assert(sizeof(chd_engine::stage_execs) / sizeof(uint64_t) == EP_COUNT, "one execution counter per stage epoch");
 
 // ---- helpers shared by the translation units (C linkage only so that definitions may sit inside their extern "C" blocks)
 extern "C" {

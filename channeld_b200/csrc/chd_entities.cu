@@ -300,6 +300,7 @@ chd_status chd_assign_cells_impl(chd_engine* e) {
         e->have_prev_key = true;
         e->assign_bump = nullptr;  // consumed
     }
+    e->assigned_since_build = true;  // (cleared by chd_build once the cell CSR matches the keys again)
     e->n_halo = 0;
     e->assigned = true;
     return CHD_OK;
@@ -440,6 +441,7 @@ chd_status chd_build(chd_engine* e) {
     if (!counts_recorded) CU(e, cudaEventRecord(e->ev_counts, e->stream));  // (cell counts final = build done)
     e->n_sorted = e->n_own + e->n_halo;
     e->built = true;
+    e->assigned_since_build = false;
     e->entities_dirty = false;
     return CHD_OK;
 }

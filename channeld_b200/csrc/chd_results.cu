@@ -481,7 +481,15 @@ chd_status chd_device_view(chd_engine* e, int which, void** d_ptr, uint64_t* cou
         case CHD_VIEW_VIS_OFF: p = e->d_vis_off; c = (uint64_t)e->n_slots + 1; break;
         case CHD_VIEW_VIS_ENTITY: p = e->d_vis; c = e->lim.max_visible; break;
         case CHD_VIEW_DUE: p = e->d_due; c = e->lim.max_due; break;
+        case CHD_VIEW_ENTER_OFF: p = e->vd.d_enter_off; c = (uint64_t)e->vd.S_out + 1; break;
+        case CHD_VIEW_ENTER_ENTITY: p = e->vd.d_enter; c = e->vd.cap; break;
+        case CHD_VIEW_LEAVE_OFF: p = e->vd.d_leave_off; c = (uint64_t)e->vd.S_out + 1; break;
+        case CHD_VIEW_LEAVE_ENTITY: p = e->vd.d_leave; c = e->vd.cap; break;
         default: return CHD_ERR_INVALID;
+    }
+    if (which >= CHD_VIEW_ENTER_OFF && !e->vd.on) {
+        e->fail("chd_device_view: the visibility delta is not enabled");
+        return CHD_ERR_STATE;
     }
     *d_ptr = p;
     if (count) *count = c;

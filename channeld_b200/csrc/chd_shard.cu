@@ -65,6 +65,7 @@ chd_status chd_set_slab(chd_engine* e, uint32_t col_lo, uint32_t col_hi, uint32_
     e->g.col_lo = col_lo;
     e->g.col_hi = col_hi;
     e->g.halo = halo;
+    e->slab_set = true;
     e->halo_on_device = false;  // set again by chd_import_halo
     return CHD_OK;
 }

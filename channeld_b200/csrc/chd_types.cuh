@@ -153,6 +153,15 @@ struct ScatterExtras {
     uint32_t* n_in_world;
 };
 
+// device-side state of the visibility-delta stage (chd_visdelta.cuh), one per engine
+struct VdState {
+    uint32_t n_now, S_now, P_now;     // this call: entities of the last build, subscriber slots, live pairs
+    uint32_t n_base, S_base, P_base;  // the baseline
+    uint32_t n_movers;                // entities whose cell key differs between the two states
+    uint32_t ovf;                     // the delta did not fit the output capacity: nothing written, baseline kept
+    unsigned long long n_enter, n_leave;
+};
+
 struct BcastDev {
     uint32_t n;
     const uint32_t *channel, *flags, *sender, *client;

@@ -298,6 +298,26 @@ class Engine:
             return self.get_visible_slot(slot, int(n.value))
         return out[:n.value].copy()
 
+    # ---- per-subscriber visibility deltas (chd_visible_delta)
+    def enable_visible_delta(self, cap):
+        """Allocates the baseline and cap entries for each of the enter / leave lists (call again to grow; the baseline is kept)."""
+        self._ck(self.L.chd_visible_delta_enable(self.h, int(cap)))
+
+    def visible_delta(self):
+        """Enqueues the delta since the previous call (stream-ordered, no host synchronisation)."""
+        self._ck(self.L.chd_visible_delta(self.h))
+
+    def get_visible_delta(self):
+        """-> (enter_off[S+1], enter_entity[], leave_off[S+1], leave_entity[]) of the last visible_delta, as numpy arrays.
+        Raises ChdError (ERR_CAPACITY) if that call overflowed its capacity."""
+        _, n_off = self.device_view(capi.VIEW_ENTER_OFF)
+        eo, lo = np.zeros(n_off, np.uint64), np.zeros(n_off, np.uint64)
+        ne, nl = C.c_uint64(), C.c_uint64()
+        self._ck(self.L.chd_get_visible_delta(self.h, ptr(eo), None, 0, ptr(lo), None, 0, C.byref(ne), C.byref(nl)))
+        ee, le = np.zeros(ne.value, np.uint32), np.zeros(nl.value, np.uint32)
+        self._ck(self.L.chd_get_visible_delta(self.h, None, ptr(ee), ne.value, None, ptr(le), nl.value, None, None))
+        return eo, ee, lo, le
+
     def get_due(self, n_due):
         out = np.zeros(int(n_due), capi.DUE_DTYPE)
         if n_due:

@@ -256,6 +256,29 @@ class GpuStaticGrid2DSpatialController {
         return r;
     }
 
+    // Per-subscriber visibility deltas (chd_visible_delta): the entities that entered / left each slot's view since the last
+    // call, CSR by slot.  The host spawns + subscribes the entity channels of `enter` and despawns + unsubscribes those of
+    // `leave` (spatial.go:797-857).
+    struct VisibleDelta {
+        std::vector<uint64_t> enter_off, leave_off;
+        std::vector<uint32_t> enter, leave;
+    };
+    void EnableVisibleDelta(uint64_t cap_entries) { check(chd_visible_delta_enable(engine_, cap_entries)); }
+    void VisibleDeltaAsync() { check(chd_visible_delta(engine_)); }
+    VisibleDelta GetVisibleDelta() {
+        void* p = nullptr;
+        uint64_t n_off = 0, ne = 0, nl = 0;
+        check(chd_device_view(engine_, CHD_VIEW_ENTER_OFF, &p, &n_off));
+        VisibleDelta r;
+        r.enter_off.resize(n_off);
+        r.leave_off.resize(n_off);
+        check(chd_get_visible_delta(engine_, r.enter_off.data(), nullptr, 0, r.leave_off.data(), nullptr, 0, &ne, &nl));
+        r.enter.resize(ne);
+        r.leave.resize(nl);
+        check(chd_get_visible_delta(engine_, nullptr, r.enter.data(), ne, nullptr, r.leave.data(), nl, nullptr, nullptr));
+        return r;
+    }
+
     chd_engine* engine() { return engine_; }
 
    private:

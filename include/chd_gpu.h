@@ -376,9 +376,46 @@ chd_status chd_fetch_wait(chd_engine* e, chd_tick_summary* summary);
 /* Device-resident views (valid until the next call that rewrites them) for consumers that stay on the GPU. */
 enum {
     CHD_VIEW_CELL_START = 0, CHD_VIEW_SORTED_ENTITY, CHD_VIEW_ENT_CELL, CHD_VIEW_PAIR_OFF, CHD_VIEW_PAIR_CHANNEL,
-    CHD_VIEW_PAIR_DIST, CHD_VIEW_VIS_OFF, CHD_VIEW_VIS_ENTITY, CHD_VIEW_DUE
+    CHD_VIEW_PAIR_DIST, CHD_VIEW_VIS_OFF, CHD_VIEW_VIS_ENTITY, CHD_VIEW_DUE,
+    /* the lists of the last chd_visible_delta (CHD_ERR_STATE before chd_visible_delta_enable): offsets count = S + 1, entity
+     * lists count = cap_entries */
+    CHD_VIEW_ENTER_OFF, CHD_VIEW_ENTER_ENTITY, CHD_VIEW_LEAVE_OFF, CHD_VIEW_LEAVE_ENTITY
 };
 chd_status chd_device_view(chd_engine* e, int which, void** d_ptr, uint64_t* count);
+
+/* ---- per-subscriber visibility deltas: the entities that entered and left each subscriber's view since the last call, without
+ * the expanded visible list (a channeld host spawns / despawns and subscribes / unsubscribes entity channels from them; the
+ * reference does this bookkeeping by hand in Notify, spatial.go:776-857).
+ *   V(s)  = { e : cell(e) in C(s) } for subscriber slot s, where cell(e) is the cell of entity e in the last chd_build (entities out
+ *           of the world and entities with id >= n are in no cell) and C(s) the slot's spatial subscriptions after the last interest
+ *           update (the pairs of chd_get_pairs): exactly the list chd_emit_visible writes for s.
+ *   The engine keeps a BASELINE: cell(e) and C(s) as they stood at the last successful chd_visible_delta (before the first call:
+ *   empty, no entity is visible to anyone).  chd_visible_delta computes for every slot
+ *           enter(s) = V_now(s) \ V_base(s)        leave(s) = V_base(s) \ V_now(s)
+ *   and makes "now" the baseline.  The delta spans everything since the previous call however many ticks that is: an entity
+ *   that left and came back in between is in neither list.
+ *   Output: two CSRs by slot, enter_off[S+1] (u64) / enter_entity[] and leave_off[S+1] / leave_entity[], S = the current slot
+ *   count (or the baseline's, if chd_set_subscribers made it smaller since: those slots' views leave too).  Fixed order: enter
+ *   entries by (current cell asc, entity id asc), leave entries by (baseline cell asc, entity id asc) within a slot.
+ *   Slots are the unit: chd_remove_subscribers / chd_set_subscribers make a slot's whole view leave, a query that errors keeps
+ *   the slot's subscriptions and so gives it no delta from them; a slot recycled between two calls (removed, then added for
+ *   another connection) shows ONE merged delta of the old and the new view.
+ *   Independent of CHD_TICK_EMIT: a tick without the expanded list gives the same delta.
+ *   Single engine only: CHD_ERR_STATE after chd_set_slab / chd_comm_init / chd_set_entity_ids (entity indices are not stable
+ *   across ticks there), also while a chd_begin_interest is pending and when cells were assigned after the last chd_build.
+ * Overflow is transactional: if either list needs more than cap_entries, the offsets are valid, the entity lists are not written
+ * and the baseline is NOT advanced (decided on the device, in stream order); chd_visible_delta_enable with the required size and
+ * another chd_visible_delta give the whole delta since the old baseline.  Nothing here touches chd_tick_summary. */
+/* allocates the baseline + output buffers (cap_entries each for enter and leave); may be called again to grow them, the baseline
+ * is kept.  Nothing is allocated on the delta path afterwards. */
+chd_status chd_visible_delta_enable(chd_engine* e, uint64_t cap_entries);
+/* stream-ordered, no host synchronisation; CHD_ERR_STATE before enable / before a build / on a sharded engine */
+chd_status chd_visible_delta(chd_engine* e);
+/* synchronous getter in the style of chd_get_visible; any pointer may be NULL; *n_enter / *n_leave = exact totals.
+ * CHD_ERR_CAPACITY if the last chd_visible_delta did not fit cap_entries or the caller's caps. */
+chd_status chd_get_visible_delta(chd_engine* e, uint64_t* enter_off, uint32_t* enter_entity, uint64_t enter_cap,
+                                 uint64_t* leave_off, uint32_t* leave_entity, uint64_t leave_cap,
+                                 uint64_t* n_enter, uint64_t* n_leave);
 
 /* ---- multi-GPU X-slab sharding (SURVEY.md §8e).  The engine owns grid columns [col_lo, col_hi) and serves
  * queries whose cells lie in [col_lo-halo, col_hi+halo).  After chd_build, chd_export_border writes the
