@@ -45,6 +45,10 @@ __global__ void __launch_bounds__(256)
         }
     }
     const uint64_t V = voff[n];
+    // A visible overflow writes no list, so no tile is described.  This is also what keeps the loop below in bounds: max_tiles
+    // counts the smaller 1024-entry warp tiles of vis_cap, while desc and general_tiles hold the 4096-entry CTA tiles of vis_cap
+    // (+8); with V > vis_cap the CTA tiles below V would write up to three times those buffers' size past their end.
+    if (V > vis_cap) return;
     for (uint64_t p = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; p < n; p += (uint64_t)gridDim.x * blockDim.x) {
         const uint64_t b = voff[p], e = voff[p + 1];
         if (e == b) continue;

@@ -335,6 +335,34 @@ def test_handover_shape(chd, oracle):
     e.close()
 
 
+@pytest.mark.parametrize("name", ["benchmark", "handover"])  # 225 cells (one radix pass per mover sort) and 65536 (two)
+def test_moving_crowd_with_a_large_entity_capacity(chd, oracle, name):
+    """A crowd of 80 % of the entities, spread over 2 x 2 cells, moves one cell along x per tick for 4 ticks: most movers share a
+    few destination (and source) cells.  max_entities > 2^21, so the mover sorts take the build's shared-memory scatter."""
+    N, S = 100_000, 128
+    wc, ex, ez = _world(chd, name, N, S)
+    rng = np.random.default_rng(3)
+    crowd = rng.uniform(size=N) < 0.8
+    ex = np.where(crowd, wc.offx + (3.0 + rng.uniform(0.01, 1.99, N)) * wc.w, ex)
+    ez = np.where(crowd, wc.offz + (3.0 + rng.uniform(0.01, 1.99, N)) * wc.h, ez)
+    e = _engine(chd, wc, (2 << 20) + 4099, S, 1 << 23)
+    base = np.zeros(0, np.uint64)
+    for tick in range(5):
+        if tick:
+            ex = np.where(crowd, ex + wc.w, ex)
+        cx, cz, r = _follow(wc, ex, ez, S)
+        now, w = _oracle_keys(oracle, wc, ex, ez, cx, cz, r)
+        assert (w["status"] == 0).all()
+        _tick(chd, e, ex, ez, cx, cz, r, (tick + 1) * 33 * MS)
+        e.visible_delta()
+        got = e.get_visible_delta()
+        _check(got, _expected(now, base, S), "tick %d" % tick)
+        if tick:
+            assert len(got[1]) > 0 and len(got[3]) > 0
+        base = now
+    e.close()
+
+
 def test_enabled_delta_changes_no_other_result(chd):
     wc, ex, ez = _world(chd, "benchmark", 30_000, 3_000)
     S = wc.n_subscribers
